@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py — rasterizer fwd+bwd frames/s on the BASELINE.json workload, one process per GPU.
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl sgr|reference] [--workload C|B|E|A]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl sgr|reference] [--workload C|B|E|A] [--dump-outputs DIR]
 
 A "step" = one forward + backward pass of the rasterizer over one synthetic frame (config C of BASELINE.md by default:
 1.5M background + 8x50k vehicle Gaussians, 1920x1280, SH degree 3).  Prints ONE JSON line (rank 0).
@@ -11,10 +11,13 @@ A "step" = one forward + backward pass of the rasterizer over one synthetic fram
                host->device (double-buffered on a copy stream) and reads the scalar loss back device->host
   roofline   : dominant kernel (blend_bwd), algorithmic bytes / CUDA-event time / measured HBM peak (MEASURED_PEAKS.json)
   cpu_baseline: the CPU oracle port (oracle/sgr_oracle.c, OpenMP) on a bounded sample of the same frame
-  --impl reference : the UNMODIFIED reference CUDA rasterizer built from /root/reference sources into oracle/_ref
+  --impl reference : the UNMODIFIED reference CUDA rasterizer built from the reference's sources into oracle/_ref
                (stock code path through its own Python API), same workload/metric/timing; the reference has no CPU
                implementation of this path, so the CPU port is reported beside it in cpu_baseline.  If oracle/_ref is
                absent the arm times the CPU oracle port instead.
+  --dump-outputs DIR : after the timed steps, what the last of them returned to the caller (images, radii, the gradient of
+               every input) as DIR/<name>.npy, float32 (indices float64); larger outputs as a fixed seeded sample.  The inputs
+               are seeded, so two builds (or the two --impl arms) can be compared output for output.
 N > 1: strong scaling — the SAME frame is tile-row sharded across ranks (street_gaussians_b200.sharded), one NCCL
 all-reduce of the per-Gaussian screen-space gradient sums per step.
 """
@@ -69,7 +72,39 @@ def parse():
     ap.add_argument("--no-clock-sampler", action="store_true")
     ap.add_argument("--diag", action="store_true", help="per-rank host/all-reduce timing breakdown on stderr")
     ap.add_argument("--cpu-sample-stride", type=int, default=0, help="CPU baseline uses every k-th Gaussian (0 = auto)")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the outputs of the last timed step to DIR/<name>.npy (single GPU; at most 64 MB, larger outputs sampled)")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    return args
+
+
+DUMP_PIXELS, DUMP_GAUSSIANS = 1 << 20, 1 << 16  # sample sizes: 5 image channels + 63 floats per Gaussian + indices stay under 64 MB
+
+
+def dump_outputs(out_dir, color, radii, depth, alpha, params, means2D):
+    """The outputs of one step as out_dir/<name>.npy: images, radii and the gradients of every input.  Images with more than
+    DUMP_PIXELS pixels are sampled at a fixed seeded set of pixels (pixel_index.npy), per-Gaussian arrays with more than
+    DUMP_GAUSSIANS rows at a fixed seeded set of Gaussians (gaussian_index.npy), so that the files stay under 64 MB."""
+    os.makedirs(out_dir, exist_ok=True)
+    dev = color.device
+    H, W = color.shape[1:]
+    P = radii.shape[0]
+    rng = np.random.default_rng(0)
+    pix = np.sort(rng.choice(H * W, DUMP_PIXELS, replace=False)) if H * W > DUMP_PIXELS else np.arange(H * W)
+    rows = np.sort(rng.choice(P, DUMP_GAUSSIANS, replace=False)) if P > DUMP_GAUSSIANS else np.arange(P)
+    pix_t, rows_t = torch.from_numpy(pix).to(dev), torch.from_numpy(rows).to(dev)
+    out = {name: img.detach().reshape(img.shape[0], -1).index_select(1, pix_t) for name, img in (("color", color), ("depth", depth), ("alpha", alpha))}
+    out["radii"] = radii.index_select(0, rows_t)
+    out.update({"grad_" + k: p.grad.index_select(0, rows_t) for k, p in params.items()})
+    out["grad_means2D"] = means2D.grad.index_select(0, rows_t)
+    arrays = {k: v.float().cpu().numpy() for k, v in out.items()}
+    arrays.update(pixel_index=pix.astype(np.float64), gaussian_index=rows.astype(np.float64))
+    total = sum(a.nbytes for a in arrays.values())
+    assert total <= 64_000_000, f"outputs of {total} bytes exceed 64 MB"
+    for k, a in arrays.items():
+        np.save(os.path.join(out_dir, k + ".npy"), a)
 
 
 class ClockSampler:
@@ -381,6 +416,9 @@ def main():
     torch.cuda.set_device(local_rank)
     dev = torch.device("cuda", local_rank)
     use_dist = world > 1 and args.impl == "sgr"
+    if use_dist and args.dump_outputs:
+        print(json.dumps({"error": "--dump-outputs writes the outputs of one process: run it with --gpus 1"}))
+        return 1
     if use_dist:
         dist.init_process_group("nccl", device_id=dev)
 
@@ -472,7 +510,7 @@ def main():
                 if gl.shape[0] < chunk:
                     gl = torch.cat([gl, gl.new_zeros((chunk - gl.shape[0],) + tuple(gl.shape[1:]))])
                 dist.all_gather_into_tensor(full_grads[k].view(-1), gl.contiguous().view(-1))
-        return color, radii
+        return color, radii, depth, alpha
 
     full_grads = {k: torch.empty((chunk * world,) + tuple(params[k].shape[1:]), device=dev) for k in PARAM_KEYS} if literal else None
 
@@ -538,7 +576,7 @@ def main():
             l0 = int(_sgr_capi.lib().sgr_launch_count())
             graph = torch.cuda.CUDAGraph()
             with torch.cuda.graph(graph):
-                color, radii = step()
+                outputs = step()
             launches_per_replay = int(_sgr_capi.lib().sgr_launch_count()) - l0
             for _ in range(3):
                 graph.replay()
@@ -570,11 +608,14 @@ def main():
         if graph is not None:
             graph.replay()
         else:
-            color, radii = step()
+            outputs = step()
         diag["host"].append((time.perf_counter() - t_h) * 1e3)
     e1.record()
     barrier()
     ms_total = e0.elapsed_time(e1)
+    color, radii = outputs[:2]
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, *outputs, params, means2D)
     # kernels of libsgr.so enqueued by THIS rank inside the timed region (counted in the library at launch / capture time; cub's sort
     # and scan kernels excluded)
     if ref_cuda:

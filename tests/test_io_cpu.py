@@ -4,11 +4,9 @@ import os
 import struct
 
 import numpy as np
-import pytest
 import torch
 
 import compose_case as CC
-import refharness as H
 from street_gaussians_b200 import io as sio
 
 
@@ -74,18 +72,18 @@ def test_checkpoint_keys_match_reference(tmp_path):
     assert torch.equal(back["obj_001"]["features_dc"], ms["obj_001"]["features_dc"]) and back["background"]["spatial_lr_scale"] == 3.5
 
 
-@pytest.mark.skipif(not H.available() or torch.cuda.is_available(), reason="needs /root/reference (build container only)")
 def test_attribute_order_and_rows_equal_the_reference_model():
-    """The reference's own GaussianModel.construct_list_of_attributes / make_ply on the same parameters (imported unmodified)."""
-    ns = H.load()
-    model = H.make_street_model(ns, n_bkgd=11, n_obj=1, per_obj=5)
-    for sub in (model.background, getattr(model, model.obj_list[0])):
-        assert sio.attribute_names(sub) == sub.construct_list_of_attributes()
-        ref_rows = sub.make_ply()  # structured array built by the reference
+    """The reference's own GaussianModel.construct_list_of_attributes / make_ply / state_dict(is_final=True) on the same parameters,
+    as recorded from the unmodified reference (tests/golden/callsite/ply_attributes.npz, tests/golden/make_io_golden.py)."""
+    z = np.load(os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "callsite", "ply_attributes.npz"))
+    for name in ("background", "obj"):
+        sub = {"_" + k: torch.from_numpy(z[f"{name}_{k}"]) for k in sio.RAW}
+        assert sio.attribute_names(sub) == list(z[name + "_attributes"])
+        ref_rows = z[name + "_ply"]  # structured array built by the reference
         mine = sio.make_ply(sub)
         assert mine.shape == (len(ref_rows), len(ref_rows.dtype.names))
         for j, n in enumerate(ref_rows.dtype.names):
             assert np.array_equal(mine[:, j], ref_rows[n]), n
         sd = sio.model_state_dict(sub)
-        ref_sd = sub.state_dict(is_final=True)
-        assert set(sd) == set(ref_sd) and all(sd[k] is ref_sd[k] for k in sd)
+        ref_sd = dict(e.split(":") for e in z[name + "_state_dict"])  # state_dict key -> the raw parameter it holds
+        assert set(sd) == set(ref_sd) and all(sd[k] is sub["_" + r] for k, r in ref_sd.items())

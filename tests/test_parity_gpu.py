@@ -1,7 +1,8 @@
 """GPU parity tests: the CUDA path (libsgr.so through the reference-compatible API / C ABI) against
   (1) the CPU oracle on seeded inputs at sizes the oracle finishes in seconds,
   (2) the committed golden fixtures (outputs of the unmodified reference CUDA rasterizer),
-  (3) the compiled reference itself (oracle/_ref) when it travelled to this box, incl. geomBuffer-level bit checks,
+  (3) the compiled reference: its recorded outputs on the scenes below (tests/golden/reference/, written by
+      tests/golden/make_ref_golden.py) and, where oracle/_ref is present, the reference itself; incl. geomBuffer-level bit checks,
   (4) size-independent properties at BASELINE.json's full sizes.
 Tolerances (BASELINE.json north_star): forward RGB within 1e-4, gradients within 1e-3 (max|d| / max|ref| per tensor)."""
 import ctypes as C
@@ -143,12 +144,8 @@ def test_golden_present():
     assert len(GOLDEN) >= 1
 
 
-def test_callsite_replay_vs_reference():
-    """SURVEY.md §8 a13, GPU half.  tests/golden/callsite/render_kernel.npz is the rasterizer call that the reference's UNMODIFIED
-    StreetGaussianRenderer.render_kernel made for a real StreetGaussianModel (recorded on the build container by
-    tests/golden/make_callsite_golden.py; tests/test_callsite_cpu.py pins the Python surface there).  Here the same call goes
-    through the compiled reference (oracle/_ref) and through this library: outputs and every .grad — including all three
-    columns of viewspace_points.grad — must agree to the north-star tolerances.  Without oracle/_ref the CPU oracle stands in."""
+def callsite_scene():
+    """tests/golden/callsite/render_kernel.npz with seeded upstream gradients."""
     from test_oracle_cpu import scene_from_npz
     path = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "callsite", "render_kernel.npz")
     scene = scene_from_npz(np.load(path))
@@ -156,8 +153,21 @@ def test_callsite_replay_vs_reference():
     g = torch.Generator().manual_seed(1)
     for k, c in (("grad_color", 3), ("grad_depth", 1), ("grad_alpha", 1)):
         scene[k] = torch.randn(c, H, W, generator=g) / (H * W)
+    return scene
+
+
+def test_callsite_replay_vs_reference():
+    """SURVEY.md §8 a13, GPU half.  tests/golden/callsite/render_kernel.npz is the rasterizer call that the reference's UNMODIFIED
+    StreetGaussianRenderer.render_kernel made for a real StreetGaussianModel (recorded from the reference's sources by
+    tests/golden/make_callsite_golden.py; tests/test_callsite_cpu.py pins the Python surface there).  Here the same call goes
+    through this library: outputs and every .grad — including all three columns of viewspace_points.grad — must agree to the
+    north-star tolerances with what the compiled reference computed for it (tests/golden/reference/callsite_render_kernel.npz),
+    and with the compiled reference itself (oracle/_ref) where it is present; without oracle/_ref the CPU oracle stands in."""
+    scene = callsite_scene()
+    H, W = scene["cam"]["image_height"], scene["cam"]["image_width"]
     mine = util.run_api(sgb, scene)
     assert mine["g_means2D"].shape == (scene["means3D"].shape[0], 3) and np.abs(mine["g_means2D"][:, 2]).max() > 0
+    assert util.check_fingerprint(mine, util.load_ref_golden("callsite_render_kernel"), scene) >= 5
     if util.ref_available():
         r = util.run_api(util.load_ref(), scene)
         assert_forward_close(mine, r, H * W, allow_flips=0)
@@ -169,20 +179,21 @@ def test_callsite_replay_vs_reference():
         assert_grads_close(mine, orc, tol=ORACLE_GRAD_TOL)
 
 
-needs_ref = pytest.mark.skipif(not util.ref_available(), reason="oracle/_ref (compiled reference) did not travel to this box")
+MEDIUM = [("200k_720p", dict(P=200_000, width=1280, height=720, sh_degree=3, seed=41, pose=True)),
+          ("60k_sem3", dict(P=60_000, width=1000, height=600, sh_degree=2, seed=42, pose=True, semantics=3))]
 
 
-@needs_ref
-@pytest.mark.parametrize("kw", [dict(P=200_000, width=1280, height=720, sh_degree=3, seed=41, pose=True),
-                                dict(P=60_000, width=1000, height=600, sh_degree=2, seed=42, pose=True, semantics=3)],
-                         ids=["200k_720p", "60k_sem3"])
-def test_cuda_vs_live_reference_medium(kw):
-    ref = util.load_ref()
+@pytest.mark.parametrize("name,kw", MEDIUM, ids=[m[0] for m in MEDIUM])
+def test_cuda_vs_live_reference_medium(name, kw):
+    """Against the recorded outputs of the compiled reference (tests/golden/reference/medium_*.npz) and, where oracle/_ref is
+    present, against the compiled reference itself."""
     scene = synthetic.make_scene(**kw)
     mine = util.run_api(sgb, scene)
-    r = util.run_api(ref, scene)
-    assert_forward_close(mine, r, kw["width"] * kw["height"], allow_flips=0)
-    assert_grads_close(mine, r)
+    assert util.check_fingerprint(mine, util.load_ref_golden("medium_" + name), scene) >= 5
+    if util.ref_available():
+        r = util.run_api(util.load_ref(), scene)
+        assert_forward_close(mine, r, kw["width"] * kw["height"], allow_flips=0)
+        assert_grads_close(mine, r)
 
 
 def _parse_ref_geom(buf: torch.Tensor, P: int):
@@ -204,21 +215,58 @@ def _parse_ref_geom(buf: torch.Tensor, P: int):
                 rgb=take(12 * P, np.float32, (P, 3)), tiles=take(4 * P, np.uint32, (P,)))
 
 
-@needs_ref
-def test_geometry_bitwise_vs_reference():
-    """The sort key is the raw float bits of the view depth and radius/rect are integer: these must be bit-equal to the
-    reference's GeometryState; conic / pixel position / RGB are compared in ulps."""
-    ref = util.load_ref()
-    scene = synthetic.make_scene(P=100_000, width=1280, height=720, sh_degree=3, seed=43, pose=True)
+GEOM_KW = dict(P=100_000, width=1280, height=720, sh_degree=3, seed=43, pose=True)
+GEOM_KEYS = ("depth", "xy", "conic_opacity", "rgb", "clamped")
+
+
+def reference_geometry(ref, scene):
+    """(instances rendered, color, radii, parsed GeometryState) of the reference's raw forward entry point."""
     dev = "cuda"
-    P = 100_000
+    P = scene["means3D"].shape[0]
     st = util.settings_from(ref, scene["cam"], dev)
     args = (st.bg, scene["means3D"].to(dev), torch.Tensor([]), torch.zeros(P, 0, device=dev), scene["opacities"].to(dev),
             scene["scales"].to(dev), scene["rotations"].to(dev), st.scale_modifier, torch.Tensor([]), st.viewmatrix, st.projmatrix,
             st.tanfovx, st.tanfovy, st.image_height, st.image_width, scene["shs"].to(dev), st.sh_degree, st.campos, False, False)
     n_ref, color, depth, alpha, sem, radii, geom, binning, img = ref._C.rasterize_gaussians(*args)
-    g = _parse_ref_geom(geom, P)
-    # candidate state through the C ABI
+    # (GeometryState.internal_radii is unused when the caller passes a radii tensor)
+    return int(n_ref), color.cpu().numpy(), radii.cpu().numpy(), _parse_ref_geom(geom, P)
+
+
+def reference_geometry_fingerprint(ref, scene, n_rows=512):
+    n_ref, color, radii, g = reference_geometry(ref, scene)
+    fp = util.fingerprint(dict(radii=radii, color=color), scene, n_rows=n_rows)
+    fp.update({"geom_" + k: g[k][fp["rows"]] for k in GEOM_KEYS}, n_rendered=np.int64(n_ref))
+    return fp
+
+
+def _assert_geometry_equal(rec, g):
+    """rec: this library's records of (a subset of) the visible Gaussians; g: the reference's GeometryState of the same ones."""
+    # record layout: q0 = (px, py, conic.xx, conic.xy), q1 = (conic.yy, opacity, power_min, depth), q2 = (r, g, b, clamp bits)
+    assert (rec[:, 7].view(np.uint32) == g["depth"].view(np.uint32)).all(), "view depth must be bit-equal (it is the sort key)"
+
+    def ulps(a, b):
+        a = a.astype(np.float32).view(np.int32).astype(np.int64); b = b.astype(np.float32).view(np.int32).astype(np.int64)
+        return np.abs(a - b)
+
+    assert ulps(rec[:, 0:2], g["xy"]).max() == 0, "pixel positions"
+    assert ulps(rec[:, [2, 3, 4]], g["conic_opacity"][:, :3]).max() <= 2, "conic"
+    assert (rec[:, 5] == g["conic_opacity"][:, 3]).all(), "opacity"
+    mine_rgb = rec[:, 8:11]
+    # SH colour is a 16-term signed sum: near a zero crossing a 1e-7 absolute difference is thousands of ulps, so bound
+    # the absolute error and require ulp-level agreement for (almost) all entries
+    assert np.abs(mine_rgb - g["rgb"]).max() <= 1e-6, "SH colour (abs)"
+    assert (ulps(mine_rgb, g["rgb"]) <= 4).mean() > 0.98, "SH colour (ulps)"
+    clamp = rec[:, 11].view(np.uint32)
+    assert (((clamp[:, None] >> np.arange(3)) & 1) == g["clamped"]).all()
+
+
+def test_geometry_bitwise_vs_reference():
+    """The sort key is the raw float bits of the view depth and radius/rect are integer: these must be bit-equal to the
+    reference's GeometryState; conic / pixel position / RGB are compared in ulps.  Against the recorded state of a sample of
+    the visible Gaussians (tests/golden/reference/geometry_100k.npz) and, where oracle/_ref is present, against all of them."""
+    scene = synthetic.make_scene(**GEOM_KW)
+    dev = "cuda"
+    P = GEOM_KW["P"]
     from street_gaussians_b200 import rasterizer as R
     mst = util.settings_from(sgb, scene["cam"], dev)
     with torch.no_grad():
@@ -227,30 +275,21 @@ def test_geometry_bitwise_vs_reference():
                                                            None, mst, None)
     torch.cuda.synchronize()
     rec = fst.geom[:P * 48].cpu().numpy().view(np.float32).reshape(P, 12)
-    ref_radii = radii.cpu().numpy()  # (GeometryState.internal_radii is unused when the caller passes a radii tensor)
-    vis = ref_radii > 0
-    assert (rad.cpu().numpy() == ref_radii).all()
-    assert vis.sum() > 50_000
-    # record layout: q0 = (px, py, conic.xx, conic.xy), q1 = (conic.yy, opacity, power_min, depth), q2 = (r, g, b, clamp bits)
-    assert (rec[vis, 7].view(np.uint32) == g["depth"][vis].view(np.uint32)).all(), "view depth must be bit-equal (it is the sort key)"
-
-    def ulps(a, b):
-        a = a.astype(np.float32).view(np.int32).astype(np.int64); b = b.astype(np.float32).view(np.int32).astype(np.int64)
-        return np.abs(a - b)
-
-    assert ulps(rec[vis, 0:2], g["xy"][vis]).max() == 0, "pixel positions"
-    assert ulps(rec[vis][:, [2, 3, 4]], g["conic_opacity"][vis, :3]).max() <= 2, "conic"
-    assert (rec[vis, 5] == g["conic_opacity"][vis, 3]).all(), "opacity"
-    mine_rgb = np.stack([rec[vis, 8], rec[vis, 9], rec[vis, 10]], 1)
-    # SH colour is a 16-term signed sum: near a zero crossing a 1e-7 absolute difference is thousands of ulps, so bound
-    # the absolute error and require ulp-level agreement for (almost) all entries
-    assert np.abs(mine_rgb - g["rgb"][vis]).max() <= 1e-6, "SH colour (abs)"
-    assert (ulps(mine_rgb, g["rgb"][vis]) <= 4).mean() > 0.98, "SH colour (ulps)"
-    clamp = rec[vis, 11].view(np.uint32)
-    assert (((clamp[:, None] >> np.arange(3)) & 1) == g["clamped"][vis]).all()
-    # exact tile culling only ever REMOVES instances, and never changes the image
+    col, rad = col.cpu().numpy(), rad.cpu().numpy()
+    fp = util.load_ref_golden("geometry_100k")
+    # radii bit-equal, and exact tile culling never changes the image (assert_allclose's atol=1e-6 + rtol=1e-7 on colours <= 1)
+    util.check_fingerprint(dict(radii=rad, color=col), fp, scene, fwd_tol=1.1e-6)
+    assert fp["radii_visible"] > 50_000
+    _assert_geometry_equal(rec[fp["rows"]], {k: fp["geom_" + k] for k in GEOM_KEYS})
+    n_ref = int(fp["n_rendered"])
+    if util.ref_available():
+        n_ref, color, radii, g = reference_geometry(util.load_ref(), scene)
+        vis = radii > 0
+        assert (rad == radii).all()
+        _assert_geometry_equal(rec[vis], {k: v[vis] for k, v in g.items()})
+        np.testing.assert_allclose(col, color, atol=1e-6)
+    # exact tile culling only ever REMOVES instances
     assert fst.num_instances <= n_ref
-    np.testing.assert_allclose(col.cpu().numpy(), color.cpu().numpy(), atol=1e-6)
     print(f"instances: reference {n_ref}, this library {fst.num_instances} ({fst.num_instances / max(n_ref, 1):.2%})")
 
 
@@ -622,10 +661,27 @@ def test_edge_cases():
     assert out[0].shape == (3, 60, 100)
 
 
+VIS_KW = dict(P=20_000, width=640, height=400, sh_degree=0, seed=71, pose=True)
+
+
+def knn_points():
+    return torch.rand(300_000, 3, generator=torch.Generator().manual_seed(72)) * torch.tensor([50.0, 5.0, 80.0])
+
+
+def reference_knn_visible(ref, rk, scene):
+    """What simple-knn's distCUDA2 and the reference rasterizer's visible_filter / markVisible return, as hashes of their bits."""
+    dev = "cuda"
+    rr = ref.GaussianRasterizer(util.settings_from(ref, scene["cam"], dev))
+    r_radii, r_m2d = rr.visible_filter(scene["means3D"].to(dev), scales=scene["scales"].to(dev), rotations=scene["rotations"].to(dev))
+    out = dict(knn=rk.distCUDA2(knn_points().to(dev)), radii=r_radii, m2d_visible=r_m2d[r_radii > 0],
+               mark_visible=rr.markVisible(scene["means3D"].to(dev)))
+    return {k + "_sha256": np.array(util.sha256(v)) for k, v in out.items()}
+
+
 def test_mark_visible_filter_and_knn():
     from oracle import oracle as O
     dev = "cuda"
-    scene = synthetic.make_scene(P=20_000, width=640, height=400, sh_degree=0, seed=71, pose=True)
+    scene = synthetic.make_scene(**VIS_KW)
     st = util.settings_from(sgb, scene["cam"], dev)
     rast = sgb.GaussianRasterizer(st)
     vis = rast.markVisible(scene["means3D"].to(dev))
@@ -642,9 +698,15 @@ def test_mark_visible_filter_and_knn():
     pts = torch.randn(5000, 3) * torch.tensor([3.0, 1.0, 0.2])
     d = sgb.distCUDA2(pts.to(dev)).cpu().numpy()
     np.testing.assert_allclose(d, O.knn_mean_dist2(pts), rtol=1e-5, atol=1e-9)
+    # bit-identity with simple-knn and with the reference's visible_filter / markVisible, against their recorded bits
+    # (tests/golden/reference/knn_visible_filter.npz)
+    fp = util.load_ref_golden("knn_visible_filter")
+    big = knn_points()
+    mine = dict(knn=sgb.distCUDA2(big.to(dev)), radii=radii, m2d_visible=m2d[radii > 0], mark_visible=vis)
+    for k, v in mine.items():
+        assert util.sha256(v) == str(fp[k + "_sha256"]), f"{k} differs from the reference's"
     if util.ref_available():
         rk = util.load_ref_knn()
-        big = torch.rand(300_000, 3) * torch.tensor([50.0, 5.0, 80.0])
         a = sgb.distCUDA2(big.to(dev)).cpu().numpy()
         b = rk.distCUDA2(big.to(dev)).cpu().numpy()
         assert (a == b).all(), "distCUDA2 must be bit-identical to simple-knn"
@@ -716,16 +778,18 @@ def test_bounded_sync_free_mode():
     assert (retry["color"] == exact["color"]).all()
 
 
-@needs_ref
 def test_full_size_parity_config_C_vs_live_reference():
     """BASELINE config C (1.9 M composed Gaussians, 1920x1280, SH 3): forward RGB within 1e-4 and every gradient tensor
-    within 1e-3 of the compiled reference on identical inputs — the north-star's parity bar at the headline size."""
-    ref = util.load_ref()
+    within 1e-3 of the compiled reference on identical inputs — the north-star's parity bar at the headline size.  Against
+    the recorded outputs of the reference (tests/golden/reference/config_C.npz) and, where oracle/_ref is present, against
+    the compiled reference itself."""
     scene = synthetic.make_config("C", seed=0)
     mine = util.run_api(sgb, scene)
-    r = util.run_api(ref, scene)
-    assert_forward_close(mine, r, 1920 * 1280, allow_flips=0)
-    assert_grads_close(mine, r, tol=GRAD_TOL)
+    assert util.check_fingerprint(mine, util.load_ref_golden("config_C"), scene, grad_tol=GRAD_TOL) >= 5
+    if util.ref_available():
+        r = util.run_api(util.load_ref(), scene)
+        assert_forward_close(mine, r, 1920 * 1280, allow_flips=0)
+        assert_grads_close(mine, r, tol=GRAD_TOL)
     # semantics of the densification statistic: column 2 of the means2D gradient is a sum of absolute values
     assert (mine["g_means2D"][:, 2] >= 0).all()
     vis = mine["radii"] > 0

@@ -1,7 +1,9 @@
 """Shared helpers for the parity tests: run the candidate (libsgr.so through the reference-compatible API), the compiled
-reference (oracle/_ref, GPU) and the CPU oracle (oracle/sgr_oracle.c) on the same seeded scene."""
+reference (oracle/_ref, GPU) and the CPU oracle (oracle/sgr_oracle.c) on the same seeded scene, and compare the candidate
+with the reference outputs recorded under tests/golden/reference/ (tests/golden/make_ref_golden.py)."""
 from __future__ import annotations
 
+import hashlib
 import os
 import sys
 
@@ -13,6 +15,83 @@ if ROOT not in sys.path:
     sys.path.insert(0, ROOT)
 
 GRAD_KEYS = ["means3D", "means2D", "shs", "opacities", "scales", "rotations"]
+REF_GOLDEN = os.path.join(ROOT, "tests", "golden", "reference")
+IMAGE_KEYS = ("color", "depth", "alpha", "semantic")
+INPUT_KEYS = ("means3D", "shs", "opacities", "scales", "rotations", "semantics", "colors_precomp", "grad_color", "grad_depth",
+              "grad_alpha", "grad_semantic")
+
+
+def sha256(a) -> str:
+    if torch.is_tensor(a):
+        a = a.detach().cpu().numpy()
+    return hashlib.sha256(np.ascontiguousarray(a).tobytes()).hexdigest()
+
+
+def fingerprint(res, scene, n_pix=1024, n_rows=96, seed=0):
+    """A small record of one forward+backward result (run_api's dict) that check_fingerprint can hold a full result against:
+    radii as a hash (they must match exactly); per image a seeded pixel sample, the per-channel sums and max|.|; per gradient
+    a seeded sample of visible rows, max|.| and sum|.|; the float64 sum of every input, so that a change of the seeded
+    generators shows up as such rather than as a parity failure."""
+    rng = np.random.default_rng(seed)
+    radii = np.asarray(res["radii"], np.int32)
+    fp = dict(radii_sha256=np.array(sha256(radii)), radii_visible=np.int64((radii > 0).sum()))
+    npx = scene["cam"]["image_height"] * scene["cam"]["image_width"]
+    fp["pix"] = np.sort(rng.choice(npx, min(n_pix, npx), replace=False)).astype(np.int32)
+    for k in IMAGE_KEYS:
+        if res.get(k) is not None and np.asarray(res[k]).size:
+            a = np.asarray(res[k], np.float32).reshape(np.asarray(res[k]).shape[0], -1)
+            fp[k + "_val"], fp[k + "_sum"], fp[k + "_maxabs"] = a[:, fp["pix"]], a.sum(1, dtype=np.float64), np.float32(np.abs(a).max())
+    vis = np.flatnonzero(radii > 0)
+    fp["rows"] = np.sort(rng.choice(vis, min(n_rows, vis.size), replace=False)).astype(np.int32)
+    for k, g in res.items():
+        if k.startswith("g_") and g is not None and np.asarray(g).size:
+            g = np.asarray(g, np.float32)
+            fp[k + "_val"], fp[k + "_maxabs"], fp[k + "_l1"] = g[fp["rows"]], np.float32(np.abs(g).max()), np.abs(g).sum(dtype=np.float64)
+    for k in INPUT_KEYS:
+        if k in scene:
+            fp["in_sum_" + k] = np.float64(scene[k].double().sum())
+    return fp
+
+
+def load_ref_golden(name):
+    with np.load(os.path.join(REF_GOLDEN, name + ".npz")) as z:
+        return {k: z[k] for k in z.files}
+
+
+def check_fingerprint(res, fp, scene, fwd_tol=1e-4, grad_tol=1e-3):
+    """Holds a full result against a recorded fingerprint with the bars of a full comparison (no pixel above fwd_tol, every
+    gradient within grad_tol * max|ref|) on the sampled entries, and with the consequences of those bars that the whole tensors
+    must meet: bit-equal radii, per-channel image sums within npx * fwd_tol, max|.| and sum|.| of every gradient within
+    grad_tol * max|ref| and numel * grad_tol * max|ref|."""
+    for k in INPUT_KEYS:
+        if "in_sum_" + k in fp:
+            got = float(scene[k].double().sum())
+            assert abs(got - float(fp["in_sum_" + k])) <= 1e-9 * max(1.0, abs(got)), f"input {k} differs from the recorded one: regenerate"
+    radii = np.asarray(res["radii"], np.int32)
+    assert sha256(radii) == str(fp["radii_sha256"]), f"radii differ ({int((radii > 0).sum())} visible, reference {int(fp['radii_visible'])})"
+    pix = fp["pix"]
+    for k in IMAGE_KEYS:
+        if k + "_val" not in fp:
+            continue
+        a = np.asarray(res[k], np.float64).reshape(fp[k + "_val"].shape[0], -1)
+        npx = a.shape[1]
+        scale = max(1.0, float(fp[k + "_maxabs"])) if k == "depth" else 1.0  # depth is un-normalised metres
+        d = np.abs(a[:, pix] - fp[k + "_val"])
+        assert d.max() <= fwd_tol * scale, (k, float(d.max()))
+        assert (np.abs(a.sum(1) - fp[k + "_sum"]) <= fwd_tol * scale * npx).all(), (k, a.sum(1), fp[k + "_sum"])
+    rows, n = fp["rows"], 0
+    for key in fp:
+        if not (key.startswith("g_") and key.endswith("_val")):
+            continue
+        k = key[:-4]
+        g = np.asarray(res[k], np.float64)
+        ref_max = float(fp[k + "_maxabs"]) + 1e-12
+        e = float(np.abs(g[rows] - fp[key]).max()) / ref_max
+        assert e <= grad_tol, (k, e)
+        assert abs(float(np.abs(g).max()) - ref_max) <= grad_tol * ref_max, (k, float(np.abs(g).max()), ref_max)
+        assert abs(float(np.abs(g).sum()) - float(fp[k + "_l1"])) <= grad_tol * ref_max * g.size, (k, float(np.abs(g).sum()), float(fp[k + "_l1"]))
+        n += 1
+    return n
 
 
 def ref_available() -> bool:
